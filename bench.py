@@ -2,6 +2,7 @@
 """bench.py -- the measurement contract.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload all|q6|sum|q1|bruteforce|ivf|dropin]
+                    [--dump-outputs DIR]
 
 The default run covers ALL FIVE BASELINE.json configs in one JSON line.  The headline (top-level keys) is config 2, TPC-H Q6
 (3-predicate filter + SUM, fp64) over SF100 synthetic lineitem columns (600 037 902 rows, 28 B/row = 16.8 GB) on one B200; the other
@@ -17,6 +18,8 @@ configs are under "workloads": sum (config 1), q1 (config 3), bruteforce (config
   cpu_baseline the oracle port (C restatement of the Go operator chain) on the host cores, bounded sample, median of 5
   parity       GPU result vs the oracle on the same rows / queries, computed in this run
   --impl reference   times that CPU implementation alone (rank 0), same metric / config / unit
+  --dump-outputs DIR writes what the last timed step of each workload returned to its caller as DIR/<workload>_<name>.npy (rank 0), so that
+                     two builds can be compared output for output: the inputs are seeded, identical from run to run
 
 Multi-GPU (one process per GPU, torchrun): q6 and sum are WEAK scaling (every rank owns an SF100-sized / 10 M-row disjoint block range),
 q1 is STRONG scaling of ONE SF100 table (shard.block_range, BASELINE config 3), bruteforce shards the 1 M rows, ivf shards the
@@ -144,6 +147,27 @@ def ncu_traffic(key):
         return (float(e["bytes_per_launch"]), e.get("source")) if e else (None, None)
     except Exception:
         return None, None
+
+
+DUMP_ARRAY_BYTES = 8 << 20     # per array: every workload together stays far below 64 MB
+
+
+def dump_outputs(out_dir, arrays):
+    """name -> array, written as out_dir/<name>.npy in float32 (float32 arrays) or float64.  64-bit integers that float64 cannot hold
+    exactly become [..., (high 32 bits, low 32 bits)].  An array above DUMP_ARRAY_BYTES keeps a fixed, seeded sample of its rows, whose
+    indices go to <name>_rows.npy."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        a = np.asarray(a)
+        if a.dtype.kind in "iub" and a.dtype.itemsize == 8 and a.size and (int(a.max()) >= 2 ** 53 or int(a.min()) <= -2 ** 53):
+            w = a.view(np.uint64)
+            a = np.stack([w >> np.uint64(32), w & np.uint64(0xFFFFFFFF)], axis=-1)
+        a = a if a.dtype == np.float32 else a.astype(np.float64)
+        if a.nbytes > DUMP_ARRAY_BYTES:
+            rows = np.sort(np.random.default_rng(0).choice(a.shape[0], max(1, DUMP_ARRAY_BYTES * a.shape[0] // a.nbytes), replace=False))
+            np.save(os.path.join(out_dir, name + "_rows.npy"), rows.astype(np.float64))
+            a = a[rows]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def median_time(fn, reps=5, warm=1):
@@ -364,8 +388,9 @@ class Env:
         self.check(self.lib.MoB200_Memset(b.ptr, 0, max(nbytes, 8)))
         return b.ptr, b
 
-    def timed(self, step, K=None, W=None):
-        """W warm-up steps, then EXACTLY K steps between CUDA events on the library stream, barrier + synchronise on both sides"""
+    def timed(self, step, K=None, W=None, outputs=None):
+        """W warm-up steps, then EXACTLY K steps between CUDA events on the library stream, barrier + synchronise on both sides.
+        outputs() is called right after the K-th step has completed: what the last timed step returned, as {name: array}"""
         K = K or self.K
         W = self.W if W is None else W
         for _ in range(W):
@@ -384,6 +409,7 @@ class Env:
         self.check(self.lib.MoB200_TimerStop(C.byref(ms)))
         self.barrier_sync()
         wall_ms = (time.perf_counter() - t_wall0) * 1e3
+        out = outputs() if outputs is not None else {}
         t_region1 = time.time()
         launches = self.lib.MoB200_KernelLaunchCount() - launches0
         total_ms = self.max_over_ranks(max(ms.value, 0.0))
@@ -400,7 +426,8 @@ class Env:
             clocks = self.sampler.window(t_region0, t_region1)
         if self.dist is not None:
             self.barrier_sync()
-        return {"total_ms": total_ms, "ms_per_step": total_ms / K, "launches": int(launches), "wall_ms": wall_ms, "clocks": clocks, "steps": K, "warmup": W}
+        return {"total_ms": total_ms, "ms_per_step": total_ms / K, "launches": int(launches), "wall_ms": wall_ms, "clocks": clocks, "steps": K, "warmup": W,
+                "outputs": out}
 
     def kernel_ms(self, step, reps=5):
         """CUDA-event duration of the dominant kernel: mean over `reps` single steps (MoB200_LastKernelMs synchronises on the kernel's
@@ -452,7 +479,7 @@ def run_q6(env, n=None):
         else:
             env.check(lib.MoB200_DownloadAsync(host.ptr, part_ptr, 16))
 
-    t = env.timed(step)
+    t = env.timed(step, outputs=lambda: {"q6_revenue": host.array[:1].copy(), "q6_rows": host.array.view(np.int64)[1:2].copy()})
     final = (float(host.array[0]), int(host.array.view(np.int64)[1]))
     # cross-check of the device seam against the synchronous API + the host-side merge (shard.py; covered by the gloo CPU test)
     sres = ops.q6_filter_sum(bufs["shipdate"], bufs["discount"], bufs["quantity"], bufs["extendedprice"], n, *P)
@@ -586,7 +613,7 @@ def run_sum(env):
         else:
             env.check(lib.MoB200_DownloadAsync(host.ptr, part_ptr, 24))
 
-    t = env.timed(step, K=max(env.K, 200))      # a 12-25 us launch: more steps for a stable figure (reported in the line)
+    t = env.timed(step, outputs=lambda: {"sum_state": host.array.view(np.int64).copy()})
     it[0] = 0
     kern_ms = env.kernel_ms(step, reps=8)
     value = n * world * t["steps"] / (t["total_ms"] * 1e-3)
@@ -652,7 +679,9 @@ def run_q1(env):
         else:
             env.check(lib.MoB200_DownloadAsync(host.ptr, part_ptr, RB))
 
-    t = env.timed(step)
+    q1_fields = ("returnflag", "linestatus", "first_row", "sum_qty", "sum_base_price", "sum_disc_price", "sum_charge", "avg_qty", "avg_price", "avg_disc",
+                 "sum_disc", "count_order")
+    t = env.timed(step, outputs=lambda: {"q1_groups": np.array([[g[f] for f in q1_fields] for g in ops.q1_result_from_bytes(host.array.tobytes())], dtype=np.float64)})
     final = ops.q1_result_from_bytes(host.array.tobytes())
     # cross-check: synchronous API + host-side merge (shard.merge_q1) must give the same groups
     sres = ops.q1_group_agg(bufs["shipdate"], bufs["quantity"], bufs["extendedprice"], bufs["discount"], bufs["tax"], bufs["returnflag"], bufs["linestatus"], n, cut)
@@ -781,8 +810,7 @@ def run_search(env, which):
             env.check(lib.MoB200_DownloadAsync(hk.ptr, kd.ptr, nq * k * 8))
             env.check(lib.MoB200_DownloadAsync(hd.ptr, dd.ptr, nq * k * 8))
 
-    t = env.timed(step)
-    final_k, final_d = hk.array.copy(), hd.array.copy()
+    t = env.timed(step, outputs=lambda: {which + "_keys": hk.array.reshape(nq, k).copy(), which + "_distances": hd.array.reshape(nq, k).copy()})
     kms = C.c_float()
     env.check(lib.MoB200_LastKernelMs(C.byref(kms)))    # the candidate pass of the last timed step
     kern_ms = kms.value
@@ -882,7 +910,7 @@ def run_dropin(env):
         da, db, dr, dn = DeviceBuffer.from_numpy(a, lib), DeviceBuffer.from_numpy(b, lib), DeviceBuffer(8 * n, lib), DeviceBuffer.from_numpy(rn, lib)
         return [Vector(data_ptr=dr.ptr, data_nbytes=8 * n, nulls_ptr=dn.ptr, length=n), Vector(data_ptr=da.ptr, data_nbytes=8 * n, length=n),
                 Vector(data_ptr=db.ptr, data_nbytes=8 * n, length=n), pv], (da, db, dr, dn)
-    out = {}
+    out, outputs = {}, {}
     for label, host in (("host_pointers", True), ("host_pointers_inputs_pinned_in_column_cache", True), ("resident", False)):
         vecs, keep = mk(host)
         if "pinned" in label:      # MoB200_ColumnPin: the block's input columns are uploaded once, later calls find them on the device
@@ -896,13 +924,15 @@ def run_dropin(env):
         for _ in range(50):
             call()
         env.sync()
-        reps = 2000
+        reps = env.K
         t0 = time.perf_counter()
         for _ in range(reps):
             rc = call()
         env.sync()
         sec = (time.perf_counter() - t0) / reps
         out[label] = {"us_per_block": sec * 1e6, "rows_per_s": n / sec, "rc": int(rc)}
+        if label == "host_pointers":
+            outputs["dropin_sum"] = keep.copy()
         if "pinned" in label:
             env.check(lib.MoB200_ColumnCacheConfigure(0))
         if host:
@@ -920,7 +950,7 @@ def run_dropin(env):
     secb = (time.perf_counter() - t0) / 5
     out["host_pointers_1024_blocks_per_call"] = {"us_per_block": secb * 1e6 / 1024, "rows_per_s": nb / secb, "rc": 0}
     ok = ok and bool(np.array_equal(R, A + B))
-    res = {"value": out["host_pointers"]["rows_per_s"], "units_per_step": n, "timing": {"total_ms": out["host_pointers"]["us_per_block"] * 2.0, "ms_per_step": out["host_pointers"]["us_per_block"] * 1e-3, "launches": 2000, "steps": 2000, "warmup": 50, "clocks": None, "wall_ms": None},
+    res = {"value": out["host_pointers"]["rows_per_s"], "units_per_step": n, "timing": {"total_ms": out["host_pointers"]["us_per_block"] * 1e-3 * env.K, "ms_per_step": out["host_pointers"]["us_per_block"] * 1e-3, "launches": env.K, "steps": env.K, "warmup": 50, "clocks": None, "wall_ms": None, "outputs": outputs},
            "kernel_ms": None, "kernel": "go_arith_kernel<int64, +>", "blocks": out, "e2e": {"value": out["host_pointers"]["rows_per_s"], "unit": "rows/s", "h2d_bytes_per_step": 16 * n, "d2h_bytes_per_step": 8 * n + n // 8, "host_memory": "pageable (numpy)"},
            "parity": {"bit_exact": ok, "ok": ok}, "parallelism": "1 OS thread, 1 block in flight"}
     if env.rank == 0 and not env.args.no_cpu:
@@ -991,6 +1021,7 @@ def main():
     ap.add_argument("--queries", type=int, default=10_000)
     ap.add_argument("--tune", action="append", default=[], metavar="NAME=VALUE",
                     help="kernel-variant knob passed to MoB200_SetTuning (experiments only; the default run uses none)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step of each workload returned as DIR/<name>.npy")
     args = ap.parse_args()
     if args.impl == "reference":
         return run_reference_arm(args)
@@ -1006,6 +1037,8 @@ def main():
         t0 = time.time()
         try:
             r = runners[w](env)
+            if args.dump_outputs and env.rank == 0:
+                dump_outputs(args.dump_outputs, r["timing"]["outputs"])
             lines[w] = finish(env, w, r)
             lines[w]["bench_seconds"] = time.time() - t0
         except Exception as ex:

@@ -21,6 +21,24 @@ def lib():
     return capi.load_library()
 
 
+@pytest.fixture(scope="module")
+def _ref_tape_store(request):
+    import ref_tape
+    name = request.module.__name__.rpartition(".")[2]
+    store = ref_tape.module_store(name)
+    yield store
+    ref_tape.write_store(name, store)
+
+
+@pytest.fixture
+def ref_tape(request, _ref_tape_store):
+    """the original's results for this test, replayed from tests/golden/ (see ref_tape.py)"""
+    import ref_tape
+    tape = ref_tape.Tape(_ref_tape_store, request.node.name)
+    yield tape
+    tape.close()
+
+
 @pytest.fixture(scope="session")
 def gpu(lib):
     from matrixone_b200 import capi

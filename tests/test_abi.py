@@ -1,6 +1,7 @@
 """C-ABI checks that need no GPU: the library loads, exports every symbol include/mo_b200.h declares, struct layouts
 match the header, and -- with no CUDA device -- every entry point FAILS LOUDLY instead of computing on the CPU."""
 import ctypes as C
+import glob
 import os
 import re
 
@@ -9,6 +10,8 @@ import pytest
 
 from matrixone_b200 import capi
 from matrixone_b200.vector import Vector, xcall
+from oracle import build as oracle_build
+from ref_tape import original
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 HEADER = os.path.join(ROOT, "include", "mo_b200.h")
@@ -30,7 +33,7 @@ def test_header_symbols_all_exported(lib):
     assert set(names) == set(capi.PROTOTYPES), set(names) ^ set(capi.PROTOTYPES)
 
 
-def test_reference_mo_h_surface_is_complete(lib):
+def test_reference_mo_h_surface_is_complete(lib, ref_tape):
     """every prototype of the reference's cgo/mo.h:24-73 (listed here by name) is exported with that exact name"""
     ref_names = ["Bitmap_Add", "Bitmap_Remove", "Bitmap_Contains", "Bitmap_IsEmpty", "Bitmap_Count", "Bitmap_And", "Bitmap_Or", "Bitmap_Not",
                  "SignedInt_VecAdd", "UnsignedInt_VecAdd", "Float_VecAdd", "SignedInt_VecSub", "UnsignedInt_VecSub", "Float_VecSub",
@@ -40,11 +43,11 @@ def test_reference_mo_h_surface_is_complete(lib):
                  "Logic_VecAnd", "Logic_VecOr", "Logic_VecXor", "Logic_VecNot", "XCall"]
     for n in ref_names:
         assert hasattr(lib, n)
-    mo_h = "/root/reference/cgo/mo.h"
-    if os.path.exists(mo_h):   # build container only: cross-check against the real header
-        src = open(mo_h).read()
-        found = re.findall(r"^\s*(?:void|bool|int32_t|uint64_t)\s+([A-Za-z_0-9]+)\s*\(", src, flags=re.M)
-        assert sorted(found) == sorted(ref_names)
+    def prototypes():    # the real header, recorded in tests/golden/ref_test_abi.npz
+        src = open(os.path.join(original(lambda: oracle_build.REF), "cgo", "mo.h")).read()
+        return np.array(re.findall(r"^\s*(?:void|bool|int32_t|uint64_t)\s+([A-Za-z_0-9]+)\s*\(", src, flags=re.M))
+    found = ref_tape(prototypes, keep=True)
+    assert sorted(found) == sorted(ref_names)
 
 
 def test_struct_layouts():
@@ -60,7 +63,7 @@ def test_version_and_launch_counter(lib):
     assert lib.MoB200_KernelLaunchCount() >= 0
 
 
-@pytest.mark.skipif(os.path.exists("/dev/nvidia0"), reason="a GPU is present; the no-device behaviour is tested on CPU boxes")
+@pytest.mark.skipif(bool(glob.glob("/dev/nvidia[0-9]*")), reason="a GPU is present; the no-device behaviour is tested on CPU boxes")
 def test_no_gpu_fails_loudly(lib):
     """no CUDA device => rc != 0 and an error text; results are never produced by a CPU path"""
     assert lib.MoB200_DeviceCount() == 0
@@ -82,7 +85,7 @@ def test_missing_library_raises_importerror(tmp_path):
         capi.load_library(str(tmp_path / "libmo_b200.so"))
 
 
-def test_bloom_header_symbols_exported_and_match_the_reference_header(lib):
+def test_bloom_header_symbols_exported_and_match_the_reference_header(lib, ref_tape):
     """include/mo_b200_bloom.h == the prototypes of the reference's cgo/bloom.h, every one exported; the host-only entry points (init, marshal,
     unmarshal, free: no GPU work) behave like cgo/bloom.c:98-135,321-339"""
     def protos(path):
@@ -92,9 +95,8 @@ def test_bloom_header_symbols_exported_and_match_the_reference_header(lib):
     assert len(names) == 18, names
     for n in names:
         assert hasattr(lib, n), n
-    ref_h = "/root/reference/cgo/bloom.h"
-    if os.path.exists(ref_h):
-        assert [n for n in protos(ref_h) if not n.startswith("bloomfilter_get_")] == names
+    ref_names = ref_tape(lambda: np.array(protos(os.path.join(original(lambda: oracle_build.REF), "cgo", "bloom.h"))), keep=True)
+    assert [n for n in ref_names if not n.startswith("bloomfilter_get_")] == names
     lib.bloomfilter_init_with_seed.restype = C.c_void_p; lib.bloomfilter_init_with_seed.argtypes = [C.c_uint64, C.c_uint32, C.c_uint64]
     lib.bloomfilter_marshal.restype = C.c_void_p; lib.bloomfilter_marshal.argtypes = [C.c_void_p, C.POINTER(C.c_size_t)]
     lib.bloomfilter_unmarshal.restype = C.c_void_p; lib.bloomfilter_unmarshal.argtypes = [C.c_void_p, C.c_size_t]

@@ -1,5 +1,6 @@
 """The bloom filter entry points of libmo_b200.so (include/mo_b200_bloom.h) against the reference's own cgo/bloom.c compiled UNCHANGED with the
-xxHash it pins (oracle/_ref/libbloom_ref.so): same results row by row and the same filter BYTES after every mutating call."""
+xxHash it pins (oracle/_ref/libbloom_ref.so, its results recorded in tests/golden/ref_test_gpu_bloom.npz): same results row by row and the
+same filter BYTES after every mutating call."""
 import ctypes as C
 import os
 
@@ -8,6 +9,7 @@ import pytest
 
 from matrixone_b200 import capi
 from matrixone_b200.vector import bitmap_from_bools, varlena_column
+from ref_tape import digest, original
 
 pytestmark = pytest.mark.gpu
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -39,9 +41,7 @@ def _proto(lib):
 @pytest.fixture(scope="module")
 def libs(gpu):
     p = os.path.join(ROOT, "oracle", "_ref", "libbloom_ref.so")
-    if not os.path.exists(p):
-        pytest.skip("oracle/_ref/libbloom_ref.so not built")
-    return _proto(capi.load_library()), _proto(C.CDLL(p))
+    return _proto(capi.load_library()), original(lambda: _proto(C.CDLL(p)) if os.path.exists(p) else None)
 
 
 def _bytes(lib, bf):
@@ -56,7 +56,7 @@ def _p(a):
 
 @pytest.mark.parametrize("dtype", [np.int8, np.int16, np.int32, np.int64, np.uint64, np.float64])
 @pytest.mark.parametrize("k,nbits", [(3, 1 << 16), (7, 100_000), (1, 64)])
-def test_fixed_add_test_and_bytes(libs, dtype, k, nbits):
+def test_fixed_add_test_and_bytes(libs, ref_tape, dtype, k, nbits):
     ours, ref = libs
     rng = np.random.default_rng(k * 131 + nbits)
     n = 20_000
@@ -64,20 +64,20 @@ def test_fixed_add_test_and_bytes(libs, dtype, k, nbits):
     keys = rng.integers(info.min, info.max, n, dtype=dtype, endpoint=True) if info else rng.standard_normal(n).astype(dtype)
     probe = np.concatenate([keys[: n // 2], (rng.integers(info.min, info.max, n // 2, dtype=dtype, endpoint=True) if info else rng.standard_normal(n // 2).astype(dtype))])
     nulls = bitmap_from_bools(rng.random(n) < 0.1)
-    a, b = ours.bloomfilter_init_with_seed(nbits, k, 12345), ref.bloomfilter_init_with_seed(nbits, k, 12345)
+    a, b = ours.bloomfilter_init_with_seed(nbits, k, 12345), ref_tape.live(lambda: ref.bloomfilter_init_with_seed(nbits, k, 12345))
     es = keys.itemsize
     ours.bloomfilter_add_fixed(a, _p(keys), keys.nbytes, es, n, _p(nulls), nulls.nbytes)
-    ref.bloomfilter_add_fixed(b, _p(keys), keys.nbytes, es, n, _p(nulls), nulls.nbytes)
-    assert _bytes(ours, a) == _bytes(ref, b)
+    ref_tape.live(lambda: ref.bloomfilter_add_fixed(b, _p(keys), keys.nbytes, es, n, _p(nulls), nulls.nbytes))
+    assert digest(_bytes(ours, a)) == ref_tape(lambda: _bytes(ref, b))
     ra, rb = np.full(n, 7, np.uint8), np.full(n, 7, np.uint8)
     ours.bloomfilter_test_fixed(a, _p(probe), probe.nbytes, es, n, _p(nulls), nulls.nbytes, _p(ra))
-    ref.bloomfilter_test_fixed(b, _p(probe), probe.nbytes, es, n, _p(nulls), nulls.nbytes, _p(rb))
-    assert (ra == rb).all()
+    _, drb = ref_tape(lambda: (ref.bloomfilter_test_fixed(b, _p(probe), probe.nbytes, es, n, _p(nulls), nulls.nbytes, _p(rb)), rb))
+    assert digest(ra) == drb
     # no nullmap: every added key is found
     ours.bloomfilter_add_fixed(a, _p(keys), keys.nbytes, es, n, None, 0)
     ours.bloomfilter_test_fixed(a, _p(keys), keys.nbytes, es, n, None, 0, _p(ra))
     assert ra.all()
-    ours.bloomfilter_free(a); ref.bloomfilter_free(b)
+    ours.bloomfilter_free(a); ref_tape.live(lambda: ref.bloomfilter_free(b))
 
 
 def test_equal_values_of_different_widths_share_their_bits(libs):
@@ -93,21 +93,21 @@ def test_equal_values_of_different_widths_share_their_bits(libs):
 
 
 @pytest.mark.parametrize("k,nbits,n", [(3, 1 << 12, 5000), (5, 1 << 20, 50_000), (2, 64, 300)])
-def test_test_and_add_keeps_the_sequential_semantics(libs, k, nbits, n):
+def test_test_and_add_keeps_the_sequential_semantics(libs, ref_tape, k, nbits, n):
     ours, ref = libs
     rng = np.random.default_rng(n)
     keys = rng.integers(0, n // 3 + 2, n, dtype=np.int64)        # many repeats: a repeat is "seen" only after its first occurrence
     nulls = bitmap_from_bools(rng.random(n) < 0.05)
-    a, b = ours.bloomfilter_init_with_seed(nbits, k, 777), ref.bloomfilter_init_with_seed(nbits, k, 777)
+    a, b = ours.bloomfilter_init_with_seed(nbits, k, 777), ref_tape.live(lambda: ref.bloomfilter_init_with_seed(nbits, k, 777))
     pre = rng.integers(0, 1000, 50, dtype=np.int64) + 10_000_000
-    ours.bloomfilter_add_fixed(a, _p(pre), pre.nbytes, 8, 50, None, 0); ref.bloomfilter_add_fixed(b, _p(pre), pre.nbytes, 8, 50, None, 0)
+    ours.bloomfilter_add_fixed(a, _p(pre), pre.nbytes, 8, 50, None, 0); ref_tape.live(lambda: ref.bloomfilter_add_fixed(b, _p(pre), pre.nbytes, 8, 50, None, 0))
     for rep in range(2):   # the second round sees the first round's bits
         ra, rb = np.full(n, 9, np.uint8), np.full(n, 9, np.uint8)
         ours.bloomfilter_test_and_add_fixed(a, _p(keys), keys.nbytes, 8, n, _p(nulls), nulls.nbytes, _p(ra))
-        ref.bloomfilter_test_and_add_fixed(b, _p(keys), keys.nbytes, 8, n, _p(nulls), nulls.nbytes, _p(rb))
-        assert (ra == rb).all(), np.flatnonzero(ra != rb)[:10]
-        assert _bytes(ours, a) == _bytes(ref, b)
-    ours.bloomfilter_free(a); ref.bloomfilter_free(b)
+        _, drb = ref_tape(lambda: (ref.bloomfilter_test_and_add_fixed(b, _p(keys), keys.nbytes, 8, n, _p(nulls), nulls.nbytes, _p(rb)), rb))
+        assert digest(ra) == drb, rep
+        assert digest(_bytes(ours, a)) == ref_tape(lambda: _bytes(ref, b))
+    ours.bloomfilter_free(a); ref_tape.live(lambda: ref.bloomfilter_free(b))
 
 
 def _rows(rng, n):
@@ -115,7 +115,7 @@ def _rows(rng, n):
     return [rng.integers(0, 256, int(l), dtype=np.uint8) for l in lens]
 
 
-def test_varlena_cells_all_length_classes(libs):
+def test_varlena_cells_all_length_classes(libs, ref_tape):
     ours, ref = libs
     rng = np.random.default_rng(5)
     n = 3000
@@ -124,52 +124,53 @@ def test_varlena_cells_all_length_classes(libs):
     probe_rows = rows[: n // 2] + _rows(rng, n - n // 2)
     pcells, parea = varlena_column(probe_rows, dtype=np.uint8)
     nulls = bitmap_from_bools(rng.random(n) < 0.1)
-    a, b = ours.bloomfilter_init_with_seed(1 << 18, 6, 4242), ref.bloomfilter_init_with_seed(1 << 18, 6, 4242)
+    a, b = ours.bloomfilter_init_with_seed(1 << 18, 6, 4242), ref_tape.live(lambda: ref.bloomfilter_init_with_seed(1 << 18, 6, 4242))
     ours.bloomfilter_add_varlena(a, _p(cells), cells.nbytes, 24, n, _p(area), area.nbytes, _p(nulls), nulls.nbytes)
-    ref.bloomfilter_add_varlena(b, _p(cells), cells.nbytes, 24, n, _p(area), area.nbytes, _p(nulls), nulls.nbytes)
-    assert _bytes(ours, a) == _bytes(ref, b)
+    ref_tape.live(lambda: ref.bloomfilter_add_varlena(b, _p(cells), cells.nbytes, 24, n, _p(area), area.nbytes, _p(nulls), nulls.nbytes))
+    assert digest(_bytes(ours, a)) == ref_tape(lambda: _bytes(ref, b))
     ra, rb = np.zeros(n, np.uint8), np.zeros(n, np.uint8)
     ours.bloomfilter_test_varlena(a, _p(pcells), pcells.nbytes, 24, n, _p(parea), parea.nbytes, _p(nulls), nulls.nbytes, _p(ra))
-    ref.bloomfilter_test_varlena(b, _p(pcells), pcells.nbytes, 24, n, _p(parea), parea.nbytes, _p(nulls), nulls.nbytes, _p(rb))
-    assert (ra == rb).all()
+    _, drb = ref_tape(lambda: (ref.bloomfilter_test_varlena(b, _p(pcells), pcells.nbytes, 24, n, _p(parea), parea.nbytes, _p(nulls), nulls.nbytes, _p(rb)), rb))
+    assert digest(ra) == drb
     ours.bloomfilter_test_and_add_varlena(a, _p(pcells), pcells.nbytes, 24, n, _p(parea), parea.nbytes, None, 0, _p(ra))
-    ref.bloomfilter_test_and_add_varlena(b, _p(pcells), pcells.nbytes, 24, n, _p(parea), parea.nbytes, None, 0, _p(rb))
-    assert (ra == rb).all() and _bytes(ours, a) == _bytes(ref, b)
-    ours.bloomfilter_free(a); ref.bloomfilter_free(b)
+    _, drb, dbytes = ref_tape(lambda: (ref.bloomfilter_test_and_add_varlena(b, _p(pcells), pcells.nbytes, 24, n, _p(parea), parea.nbytes, None, 0, _p(rb)), rb, _bytes(ref, b)))
+    assert digest(ra) == drb and digest(_bytes(ours, a)) == dbytes
+    ours.bloomfilter_free(a); ref_tape.live(lambda: ref.bloomfilter_free(b))
 
 
-def test_length_prefixed_stream_single_keys_marshal_or(libs):
+def test_length_prefixed_stream_single_keys_marshal_or(libs, ref_tape):
     ours, ref = libs
     rng = np.random.default_rng(6)
     rows = _rows(rng, 500)
     stream = np.concatenate([np.concatenate([np.array([len(r)], np.uint32).view(np.uint8), r]) for r in rows])
-    a, b = ours.bloomfilter_init_with_seed(1 << 15, 3, 1), ref.bloomfilter_init_with_seed(1 << 15, 3, 1)
-    ours.bloomfilter_add_varlena_4b(a, _p(stream), stream.nbytes, 500, None, 0); ref.bloomfilter_add_varlena_4b(b, _p(stream), stream.nbytes, 500, None, 0)
-    assert _bytes(ours, a) == _bytes(ref, b)
+    a, b = ours.bloomfilter_init_with_seed(1 << 15, 3, 1), ref_tape.live(lambda: ref.bloomfilter_init_with_seed(1 << 15, 3, 1))
+    ours.bloomfilter_add_varlena_4b(a, _p(stream), stream.nbytes, 500, None, 0); ref_tape.live(lambda: ref.bloomfilter_add_varlena_4b(b, _p(stream), stream.nbytes, 500, None, 0))
+    assert digest(_bytes(ours, a)) == ref_tape(lambda: _bytes(ref, b))
     cut = stream[: stream.nbytes - 7]     # a truncated stream: rows past the cut are not touched
     ra, rb = np.full(500, 5, np.uint8), np.full(500, 5, np.uint8)
-    ours.bloomfilter_test_varlena_4b(a, _p(cut), cut.nbytes, 500, None, 0, _p(ra)); ref.bloomfilter_test_varlena_4b(b, _p(cut), cut.nbytes, 500, None, 0, _p(rb))
-    assert (ra == rb).all()
+    ours.bloomfilter_test_varlena_4b(a, _p(cut), cut.nbytes, 500, None, 0, _p(ra))
+    _, drb = ref_tape(lambda: (ref.bloomfilter_test_varlena_4b(b, _p(cut), cut.nbytes, 500, None, 0, _p(rb)), rb))
+    assert digest(ra) == drb
     # single-key entry points
     for r in rows[:20] + [np.frombuffer(b"not there", np.uint8)]:
-        assert ours.bloomfilter_test(a, _p(r), r.nbytes) == ref.bloomfilter_test(b, _p(r), r.nbytes)
+        assert ours.bloomfilter_test(a, _p(r), r.nbytes) == ref_tape(lambda: ref.bloomfilter_test(b, _p(r), r.nbytes))
     k1 = np.frombuffer(b"a brand new key", np.uint8)
-    assert ours.bloomfilter_test_and_add(a, _p(k1), k1.nbytes) == ref.bloomfilter_test_and_add(b, _p(k1), k1.nbytes) == False
-    assert ours.bloomfilter_test_and_add(a, _p(k1), k1.nbytes) == ref.bloomfilter_test_and_add(b, _p(k1), k1.nbytes) == True
+    assert ours.bloomfilter_test_and_add(a, _p(k1), k1.nbytes) == ref_tape(lambda: ref.bloomfilter_test_and_add(b, _p(k1), k1.nbytes)) == False
+    assert ours.bloomfilter_test_and_add(a, _p(k1), k1.nbytes) == ref_tape(lambda: ref.bloomfilter_test_and_add(b, _p(k1), k1.nbytes)) == True
     k2 = np.array([123456789], np.int64)
-    ours.bloomfilter_add(a, _p(k2), 8); ref.bloomfilter_add(b, _p(k2), 8)
-    assert _bytes(ours, a) == _bytes(ref, b)
+    ours.bloomfilter_add(a, _p(k2), 8); ref_tape.live(lambda: ref.bloomfilter_add(b, _p(k2), 8))
+    assert digest(_bytes(ours, a)) == ref_tape(lambda: _bytes(ref, b))
     # marshal -> unmarshal -> probe; or
     raw = np.frombuffer(_bytes(ours, a), np.uint8).copy()
     u = ours.bloomfilter_unmarshal(_p(raw), raw.nbytes)
     assert u == raw.ctypes.data
     for r in rows[:20]:
         assert ours.bloomfilter_test(u, _p(r), r.nbytes)
-    c, d = ours.bloomfilter_init_with_seed(1 << 15, 3, 1), ref.bloomfilter_init_with_seed(1 << 15, 3, 1)
+    c, d = ours.bloomfilter_init_with_seed(1 << 15, 3, 1), ref_tape.live(lambda: ref.bloomfilter_init_with_seed(1 << 15, 3, 1))
     more = rng.integers(0, 1 << 40, 1000, dtype=np.int64)
-    ours.bloomfilter_add_fixed(c, _p(more), more.nbytes, 8, 1000, None, 0); ref.bloomfilter_add_fixed(d, _p(more), more.nbytes, 8, 1000, None, 0)
-    assert ours.bloomfilter_or(a, a, c) == ref.bloomfilter_or(b, b, d) == 0      # Merge: dst == a (cbloomfilter.go:435)
-    assert _bytes(ours, a) == _bytes(ref, b)
+    ours.bloomfilter_add_fixed(c, _p(more), more.nbytes, 8, 1000, None, 0); ref_tape.live(lambda: ref.bloomfilter_add_fixed(d, _p(more), more.nbytes, 8, 1000, None, 0))
+    assert ours.bloomfilter_or(a, a, c) == ref_tape(lambda: ref.bloomfilter_or(b, b, d)) == 0      # Merge: dst == a (cbloomfilter.go:435)
+    assert digest(_bytes(ours, a)) == ref_tape(lambda: _bytes(ref, b))
     e = ours.bloomfilter_init_with_seed(1 << 16, 3, 1)
     assert ours.bloomfilter_or(a, a, e) == 1
     f = ours.bloomfilter_init_with_seed(1 << 15, 3, 2)
@@ -179,22 +180,22 @@ def test_length_prefixed_stream_single_keys_marshal_or(libs):
     for x in (a, c, e, f, g):
         ours.bloomfilter_free(x)
     for x in (b, d):
-        ref.bloomfilter_free(x)
+        ref_tape.live(lambda: ref.bloomfilter_free(x))
 
 
-def test_device_resident_keys_and_results(libs):
+def test_device_resident_keys_and_results(libs, ref_tape):
     from matrixone_b200.vector import DeviceBuffer
     ours, ref = libs
     rng = np.random.default_rng(8)
     n = 1_000_000
     keys = rng.integers(0, 1 << 62, n, dtype=np.int64)
-    a, b = ours.bloomfilter_init_with_seed(1 << 24, 3, 5), ref.bloomfilter_init_with_seed(1 << 24, 3, 5)
+    a, b = ours.bloomfilter_init_with_seed(1 << 24, 3, 5), ref_tape.live(lambda: ref.bloomfilter_init_with_seed(1 << 24, 3, 5))
     dk = DeviceBuffer.from_numpy(keys); dr = DeviceBuffer(n)
     ours.bloomfilter_add_fixed(a, dk.ptr, keys.nbytes, 8, n // 2, None, 0)
-    ref.bloomfilter_add_fixed(b, _p(keys), keys.nbytes, 8, n // 2, None, 0)
+    ref_tape.live(lambda: ref.bloomfilter_add_fixed(b, _p(keys), keys.nbytes, 8, n // 2, None, 0))
     ours.bloomfilter_test_fixed(a, dk.ptr, keys.nbytes, 8, n, None, 0, dr.ptr)
     rb = np.zeros(n, np.uint8)
-    ref.bloomfilter_test_fixed(b, _p(keys), keys.nbytes, 8, n, None, 0, _p(rb))
-    assert (dr.to_numpy(np.uint8) == rb).all()
-    assert _bytes(ours, a) == _bytes(ref, b)
-    ours.bloomfilter_free(a); ref.bloomfilter_free(b); dk.free(); dr.free()
+    _, drb = ref_tape(lambda: (ref.bloomfilter_test_fixed(b, _p(keys), keys.nbytes, 8, n, None, 0, _p(rb)), rb))
+    assert digest(dr.to_numpy(np.uint8)) == drb
+    assert digest(_bytes(ours, a)) == ref_tape(lambda: _bytes(ref, b))
+    ours.bloomfilter_free(a); ref_tape.live(lambda: ref.bloomfilter_free(b)); dk.free(); dr.free()

@@ -1,4 +1,5 @@
-"""GPU parity: row-wise distances behind XCall.  Reference ids 0..3 against the reference C (oracle/_ref, 1e-5 relative --
+"""GPU parity: row-wise distances behind XCall.  Reference ids 0..3 against the reference C (oracle/_ref, its results recorded in
+tests/golden/ref_test_gpu_distance.npz; 1e-5 relative --
 the C accumulates in double under -ffast-math); new Go-semantics ids 100..109 BIT-EXACT against the oracle restatement
 of pkg/vectorindex/metric/distance_func.go, plus the reference's golden vectors."""
 import ctypes as C
@@ -11,6 +12,7 @@ import pytest
 import oracle_lib as O
 from matrixone_b200 import capi
 from matrixone_b200.vector import DeviceBuffer, Vector, bitmap_from_bools, varlena_column, varlena_column_from_matrix, xcall
+from ref_tape import original
 
 pytestmark = pytest.mark.gpu
 G = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
@@ -92,10 +94,8 @@ def test_cosine_similarity_zero_vector_is_an_error_and_dim_mismatch(gpu):
 
 
 @pytest.mark.parametrize("dt,ids", [(np.float32, (0, 2)), (np.float64, (1, 3))])
-def test_reference_ids_match_reference_c(gpu, dt, ids):
-    ref = O.ref()
-    if ref is None:
-        pytest.skip("oracle/_ref missing")
+def test_reference_ids_match_reference_c(gpu, ref_tape, dt, ids):
+    ref = original(O.ref)
     rng = np.random.default_rng(3)
     n, dim = 1000, 768
     a = rng.standard_normal((n, dim)).astype(dt); b = rng.standard_normal((n, dim)).astype(dt)
@@ -108,9 +108,10 @@ def test_reference_ids_match_reference_c(gpu, dt, ids):
                 va, vb = _cols(a), _cols(bb)
                 args = (capi.XCallArgs * 3)(Vector(data=r1, nulls=nulls, length=n).fill_raw_ptr_len(), va.fill_raw_ptr_len(), vb.fill_raw_ptr_len())
                 err = (C.c_uint8 * 256)()
-                assert ref.XCall(0, fid, err, C.cast(args, C.c_void_p), n) == 0
+                rc1, want = ref_tape(lambda: (ref.XCall(0, fid, err, C.cast(args, C.c_void_p), n), r1), keep=True)
+                assert rc1 == 0
                 xcall(fid, [Vector(data=r2, nulls=nulls, length=n), va, vb], n, runtime_id=1)
-                np.testing.assert_allclose(r2, r1, rtol=1e-5, atol=0)      # tolerance stated by north_star
+                np.testing.assert_allclose(r2, want, rtol=1e-5, atol=0)
                 if nulls is not None:
                     from matrixone_b200.vector import bitmap_to_bools
                     assert (r2[bitmap_to_bools(rn, n)] == -1.0).all()         # null rows are left unwritten (xcall.c:57)
