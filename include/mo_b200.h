@@ -293,6 +293,42 @@ typedef struct mo_join_params_t { int32_t join_type; int32_t reserved; } mo_join
 #define MO_XCALL_JOIN_PROBE 0x6012
 #define MO_XCALL_GROUP_AGG(op, T) (0x6400 + ((op) << 8) + (T))
 
+/* ---- group-by and hash join on keys wider than 8 bytes: the StrHashMap path (csrc/strhash.cu).  The reference takes it for any varchar / char
+ * key, any composite key wider than 8 bytes (a nullable column costs one byte more, group/exec2.go:73-94,167-188) and any join whose equality
+ * columns are wider than 8 bytes (hashbuild/hashmap.go:258-277).  A packed key table is "offsets int64[ngroups + 1] + bytes": the key of 1-based
+ * group g is bytes[offsets[g - 1] .. offsets[g]).  Everything behind the ids is shared with the 8-byte path: GROUP_AGG, DEC_SUM, JOIN_SELS.
+ * All four calls are synchronous; pointers as everywhere (host or device).
+ *   PACK_STR_KEYS   strHashmapIterator.encodeHashKeys (pkg/common/hashmap/strhashmap.go:92-385), the exact bytes.  Per column, in column order:
+ *                   fixed width w, has_null: marker 0 + the w value bytes, a NULL appends marker 1 only ; fixed, no has_null: the w value bytes,
+ *                   a NULL makes the row skip (zValues = 0) and the column appends nothing ; varlena, has_null: marker 0 + length as little-endian
+ *                   uint16 + the bytes, a NULL appends marker 1 ; varlena, no has_null: uint16 length + bytes, a NULL skips the row.  The length
+ *                   field is truncated to 16 bits, the bytes are not.  A const vector repeats element 0, a const NULL appends marker 1 (has_null)
+ *                   or skips every row.  Keys shorter than 16 bytes are zero-padded to 16 (hashtable.StrKeyPadding).
+ *                   args: [0] offsets int64[len + 1] (out; + pnulls out, no has_null mode: the rows that join no group) ; [1] key bytes (out;
+ *                   capacity = dataSz) ; [2] host mo_str_key_params_t ; [3 .. 3 + ncols) the key columns (+pnulls): fixed width = width[k] bytes
+ *                   per row (any width >= 1: Decimal128, uuid, Rowid), varlena (width 0) = 24-byte cells with parea.  A const vector holds one
+ *                   element.  When the bytes do not fit, the call fails with MO_RC_OUT_OF_RANGE and offsets[len] holds the bytes needed.
+ *   STR_GROUP_IDS   strHashmapIterator.Insert as driven by Group.buildOneBatch (exec2.go:325-362, string_hash_map.go:97-158): 1-based group ids
+ *                   in FIRST-SEEN order, 0 for a skipped row.  Two keys are one group when their bytes are equal (the reference compares 192-bit
+ *                   hash states; the ids are the same).  The table persists across calls in caller-owned buffers.
+ *                   args: [0] groups uint64[len] ; [1] state int64[4] = {ngroups (in/out), key bytes used (in/out), groups needed (out), bytes
+ *                   needed (out)} ; [2] table offsets int64[capacity + 1] ; [3] table bytes (capacity = dataSz) ; [4] packed key offsets
+ *                   int64[len + 1] (+pnulls: rows that get id 0) ; [5] packed key bytes.  More groups than the capacity or more key bytes than the
+ *                   table holds: MO_RC_OUT_OF_RANGE with state[2], state[3] set, and ngroups, bytes used and the table left unchanged; the caller
+ *                   grows its buffers and repeats the call.
+ *   STR_JOIN_FIND   strHashmapIterator.Find: vals[i] = 1-based group id of probe key i, 0 = absent, NULL or skipped.
+ *                   args: [0] vals uint64[len] ; [1] table offsets int64[ngroups + 1] ; [2] table bytes ; [3] probe key offsets (+pnulls) ; [4] probe key bytes
+ *   STR_JOIN_PROBE  JOIN_PROBE over string keys: same join types, emission order, capacity protocol and sels.  args: [0 .. 3] as JOIN_PROBE ;
+ *                   [4] table offsets ; [5] table bytes ; [6] sels offsets ; [7] sels vals ; [8] probe key offsets (+pnulls) ; [9] probe key bytes
+ * The device hash table is rebuilt from the key table per call (like GROUP_IDS) unless MoB200_StrJoinMapPrepare cached it for FIND / PROBE.
+ * Not provided here: string keys inside MO_XCALL_PLAN, the grouping-set marker 2 (ROLLUP / CUBE), non-equality join conditions, right joins. */
+#define MO_STR_KEY_MAX_COLS 16
+typedef struct mo_str_key_params_t { int32_t ncols; int32_t has_null; int32_t width[MO_STR_KEY_MAX_COLS]; /* 0 = varlena */ } mo_str_key_params_t;
+#define MO_XCALL_PACK_STR_KEYS 0x6003
+#define MO_XCALL_STR_GROUP_IDS 0x6004
+#define MO_XCALL_STR_JOIN_FIND 0x6013
+#define MO_XCALL_STR_JOIN_PROBE 0x6014
+
 /* ---- Decimal64 / Decimal128 (csrc/decimal.cu): the reference's native TPC-H column type is DECIMAL(15,2).  Decimal64 = int64 unscaled value,
  * Decimal128 = 16 bytes two's complement {B0_63, B64_127}; scales travel in the parameter block.  Conventions of the Go engine (as GO_ARITH).
  *   DEC_ARITH(op, width)  op 0 + 1 - 2 * ; width 64 / 128 = operand type.  d64Add/d64Sub/d64Mul/d128Add/d128Sub/d128Mul,
@@ -451,6 +487,10 @@ int32_t MoB200_ColumnCacheStats(uint64_t *hits, uint64_t *misses, uint64_t *byte
  * pkg/vm/message/joinMapMsg.go:127-160); JOIN_FIND / JOIN_PROBE calls whose table_keys pointer equals `table_keys` reuse it. */
 int32_t MoB200_JoinMapPrepare(const void *table_keys, uint64_t ngroups);
 int32_t MoB200_JoinMapRelease(const void *table_keys);
+/* the same for a string-keyed JoinMap (MO_XCALL_STR_JOIN_FIND / STR_JOIN_PROBE): the key table (offsets int64[ngroups + 1] + bytes) is copied to
+ * the device with its hash table; calls whose table offsets pointer equals `key_offsets` (and whose group count matches) use the prepared copy. */
+int32_t MoB200_StrJoinMapPrepare(const void *key_offsets, const void *key_bytes, uint64_t ngroups);
+int32_t MoB200_StrJoinMapRelease(const void *key_offsets);
 int32_t MoB200_Sync(void);                    /* synchronize the calling thread's stream */
 int32_t MoB200_SetStream(void *cuda_stream);  /* adopt an external cudaStream_t for the calling thread (NULL = own) */
 int32_t MoB200_TimerStart(void);              /* CUDA event on the calling thread's stream */

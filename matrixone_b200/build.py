@@ -14,7 +14,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 OUT = os.path.join(HERE, "libmo_b200.so")
 OBJ = os.path.join(HERE, "build")
-SOURCES = ["runtime.cu", "agg.cu", "tpch.cu", "elementwise.cu", "goelem.cu", "colops.cu", "join.cu", "kmeans.cu", "lz4.cu", "vecdecode.cu", "plan.cu", "decimal.cu", "bloom.cu", "distance.cu", "search.cu", "tcsearch.cu", "xcall.cu", "datagen.cu"]
+SOURCES = ["runtime.cu", "agg.cu", "tpch.cu", "elementwise.cu", "goelem.cu", "colops.cu", "join.cu", "strhash.cu", "kmeans.cu", "lz4.cu", "vecdecode.cu", "plan.cu", "decimal.cu", "bloom.cu", "distance.cu", "search.cu", "tcsearch.cu", "xcall.cu", "datagen.cu"]
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17", "-Xcompiler", "-fPIC",
          "--expt-relaxed-constexpr", "-Xptxas", "-v"]

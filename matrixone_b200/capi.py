@@ -48,6 +48,9 @@ def XCALL_AGG_MERGE(op, T):
 
 XCALL_FILTER_SELS, XCALL_PACK_KEYS, XCALL_GROUP_IDS = 0x6000, 0x6001, 0x6002
 XCALL_JOIN_SELS, XCALL_JOIN_FIND, XCALL_JOIN_PROBE = 0x6010, 0x6011, 0x6012
+XCALL_PACK_STR_KEYS, XCALL_STR_GROUP_IDS = 0x6003, 0x6004
+XCALL_STR_JOIN_FIND, XCALL_STR_JOIN_PROBE = 0x6013, 0x6014
+STR_KEY_MAX_COLS = 16
 XCALL_KMEANS_ELKAN_F32, XCALL_KMEANS_ELKAN_F64 = 0x6020, 0x6021
 XCALL_LZ4_DECODE = 0x6030
 XCALL_VECTOR_UNMARSHAL = 0x6031
@@ -99,6 +102,11 @@ class XCallArgs(C.Structure):
                 ("parea", C.c_void_p), ("areaSz", C.c_uint64)]
 
 
+class StrKeyParams(C.Structure):
+    """mo_str_key_params_t: width[k] = fixed element bytes of key column k, 0 = varlena"""
+    _fields_ = [("ncols", C.c_int32), ("has_null", C.c_int32), ("width", C.c_int32 * STR_KEY_MAX_COLS)]
+
+
 class Q6Params(C.Structure):
     _fields_ = [("date_lo", C.c_int32), ("date_hi", C.c_int32), ("disc_lo", C.c_double), ("disc_hi", C.c_double),
                 ("qty_hi", C.c_double)]
@@ -143,6 +151,7 @@ PROTOTYPES = {
     "MoB200_ColumnCacheConfigure": (_i32, [_u64]), "MoB200_ColumnPin": (_i32, [_vp, _u64, _u64]), "MoB200_ColumnUnpin": (_i32, [_vp]),
     "MoB200_ColumnCacheStats": (_i32, [C.POINTER(_u64), C.POINTER(_u64), C.POINTER(_u64)]),
     "MoB200_JoinMapPrepare": (_i32, [_vp, _u64]), "MoB200_JoinMapRelease": (_i32, [_vp]),
+    "MoB200_StrJoinMapPrepare": (_i32, [_vp, _vp, _u64]), "MoB200_StrJoinMapRelease": (_i32, [_vp]),
     "MoB200_DownloadAsync": (_i32, [_vp, _vp, _u64]), "MoB200_UploadAsync": (_i32, [_vp, _vp, _u64]),
     "MoB200_Sync": (_i32, []), "MoB200_SetStream": (_i32, [_vp]), "MoB200_TimerStart": (_i32, []),
     "MoB200_TimerStop": (_i32, [C.POINTER(C.c_float)]), "MoB200_KernelLaunchCount": (_u64, []), "MoB200_LastKernelMs": (_i32, [C.POINTER(C.c_float)]),

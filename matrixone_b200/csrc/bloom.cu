@@ -90,12 +90,7 @@ __device__ __forceinline__ bool key_of(const KeySrc &K, uint64_t i, const uint8_
     }
     if (i * K.elemsz + (K.varlena ? (uint64_t)MO_VARLENA_SZ : K.elemsz) > K.len) return false;   // the reference's  j < len  loop bound (a trailing partial element is not read)
     if (!K.varlena) { *p = K.keys + i * K.elemsz; *n = K.elemsz; return true; }
-    const uint8_t *c = K.keys + i * K.elemsz;
-    if (c[0] <= MO_VARLENA_INLINE_SZ) { *p = c + 1; *n = c[0]; return true; }
-    const uint32_t off = xxh3::rd32(c + 4), ln = xxh3::rd32(c + 8);
-    if (!K.area || (uint64_t)off + ln > K.area_len) return false;   // (the reference would read out of bounds here; such a row is skipped)
-    *p = K.area + off; *n = ln;
-    return true;
+    return varlena_bytes(K.keys + i * K.elemsz, K.area, K.area_len, p, n);   // (a big cell outside the area: the reference would read out of bounds; such a row is skipped)
 }
 
 // MODE 0: add, 1: test

@@ -12,7 +12,7 @@
 // These are what the fused plans (tpch.cu, plan.cu) are built from; exposed on their own they make every operator of the chain
 // available on resident columns.  All are HBM- or atomic-throughput bound integer/byte kernels: coalesced 128-bit loads, warp
 // ballots for bitmaps, a single-pass decoupled look-back scan for the order-preserving compaction.
-#include "common.cuh"
+#include "hashops.cuh"
 #include <cstring>
 
 using namespace mob;
@@ -106,6 +106,9 @@ select_kernel(const uint8_t *__restrict__ v, const uint64_t *__restrict__ nulls,
     for (unsigned i = threadIdx.x; i < agg; i += kSelThreads) sels[out0 + i] = (OutT)(tile_row0 + s_list[i]);
 }
 
+}  // namespace
+
+namespace mob {
 // launches the compaction; *dtotal (device) receives the count.  status/ticket scratch comes from the arena.
 template <typename OutT>
 int launch_select(ThreadCtx &t, const uint8_t *v, const uint64_t *nulls, uint64_t n, OutT *sels, unsigned long long *dtotal) {
@@ -119,6 +122,11 @@ int launch_select(ThreadCtx &t, const uint8_t *v, const uint64_t *nulls, uint64_
     MOB_LAUNCH_CHECK();
     return MO_RC_SUCCESS;
 }
+template int launch_select<int64_t>(ThreadCtx &, const uint8_t *, const uint64_t *, uint64_t, int64_t *, unsigned long long *);
+template int launch_select<uint32_t>(ThreadCtx &, const uint8_t *, const uint64_t *, uint64_t, uint32_t *, unsigned long long *);
+}  // namespace mob
+
+namespace {
 
 // =========================================================================================================
 // gather (Shrink / Union / FixedLengthShuffle) with nulls.Filter fused: dst[i] = src[sels[i]], dst null bit i = src null bit sels[i]

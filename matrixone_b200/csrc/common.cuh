@@ -126,6 +126,17 @@ __device__ __forceinline__ void st_stream16(void *p, int4 v) {
 
 __device__ __forceinline__ bool bm_test(const uint64_t *p, uint64_t i) { return p && ((p[i >> 6] >> (i & 63)) & 1ull); }
 
+// the bytes of one MatrixOne varlena cell (pkg/container/types/bytes.go:61-115): c[0] <= 23 -> inline, bytes c[1 .. 1 + c[0]); otherwise
+// uint32 offset at c + 4 and uint32 length at c + 8 into the area.  false when a big cell points outside [area, area + area_len).
+__device__ __forceinline__ bool varlena_bytes(const uint8_t *c, const uint8_t *area, uint64_t area_len, const uint8_t **p, uint64_t *n) {
+    if (c[0] <= MO_VARLENA_INLINE_SZ) { *p = c + 1; *n = c[0]; return true; }
+    const uint32_t off = (uint32_t)c[4] | ((uint32_t)c[5] << 8) | ((uint32_t)c[6] << 16) | ((uint32_t)c[7] << 24);
+    const uint32_t ln = (uint32_t)c[8] | ((uint32_t)c[9] << 8) | ((uint32_t)c[10] << 16) | ((uint32_t)c[11] << 24);
+    if (!area || (uint64_t)off + ln > area_len) return false;
+    *p = area + off; *n = ln;
+    return true;
+}
+
 template <typename T>
 __device__ __forceinline__ T warp_sum(T v) {
 #pragma unroll

@@ -14,7 +14,7 @@
 //   The hash table itself is not observable in the reference (random seeds): ids and pairs are.  The device table is rebuilt from table_keys per
 //   call (O(groups)) unless it was prepared with MoB200_JoinMapPrepare (cached per table_keys pointer).
 // All passes stream their inputs once; algorithmic bytes per probe row: 8 (key) + 16 per emitted pair + one random 8-byte table probe.
-#include "common.cuh"
+#include "hashops.cuh"
 #include <cstring>
 #include <mutex>
 #include <shared_mutex>
@@ -28,12 +28,6 @@ constexpr int kThreads = 256;
 constexpr uint64_t kEmptyKey = 0xffffffffffffffffull;
 
 __device__ __forceinline__ uint64_t mix64(uint64_t x) { x ^= x >> 33; x *= 0xff51afd7ed558ccdull; x ^= x >> 33; x *= 0xc4ceb9fe1a85ec53ull; return x ^ (x >> 33); }
-
-inline unsigned grid_for(uint64_t items, int per_block = kThreads) {
-    uint64_t g = (items + per_block - 1) / per_block;
-    const uint64_t mx = (uint64_t)num_sms() * (per_block == 1 ? 32 : 16);
-    return (unsigned)(g > mx ? mx : (g ? g : 1));
-}
 
 // ---- exclusive scan of uint64 (three kernels: tile sums, scan of the sums by one CTA, apply) ---------------------------------------------------
 constexpr int kScanTile = 2048;   // 256 threads x 8
@@ -85,6 +79,8 @@ __global__ void __launch_bounds__(kThreads) scan_apply_kernel(const uint64_t *__
     for (int w = 0; w < warp; w++) run += sw[w];
     for (int j = 0; j < 8; j++) { if (base + j < n) out[base + j] = run; run += v[j]; }
 }
+}  // namespace
+
 // out[i] = sum of in[0 .. i); *total (device) = sum of all.  in == out allowed.  sums scratch from the arena.
 int exclusive_scan(ThreadCtx &t, const uint64_t *in, uint64_t n, uint64_t *out, uint64_t *total) {
     if (n == 0) { MOB_CUDA_TRY(cudaMemsetAsync(total, 0, 8, t.stream)); return MO_RC_SUCCESS; }
@@ -99,6 +95,8 @@ int exclusive_scan(ThreadCtx &t, const uint64_t *in, uint64_t n, uint64_t *out, 
     MOB_LAUNCH_CHECK();
     return MO_RC_SUCCESS;
 }
+
+namespace {
 
 // ---- JOIN_SELS ------------------------------------------------------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(kThreads) sels_flag_kernel(const uint64_t *__restrict__ groups, uint64_t n, uint64_t ngroups, uint64_t *__restrict__ flag, uint64_t *__restrict__ cnt, unsigned *bad) {
@@ -257,18 +255,9 @@ __global__ void __launch_bounds__(kThreads) probe_count_kernel(const uint64_t *_
                                                                int join_type, uint32_t *__restrict__ vals, uint64_t *__restrict__ cnt) {
     for (uint64_t i = blockIdx.x * (uint64_t)kThreads + threadIdx.x; i < n; i += (uint64_t)gridDim.x * kThreads) {
         const bool isnull = knulls && ((knulls[i >> 6] >> (i & 63)) & 1ull);
-        const uint32_t v = isnull ? 0u : jt_find(tkey, tid, mask, sentinel_id, keys[i]);
-        uint64_t m = 0;
-        if (v) m = offsets ? (uint64_t)(offsets[v] - offsets[v - 1]) : 1ull;
-        uint64_t c;
-        switch (join_type) {
-        case MO_JOIN_INNER: c = m; break;
-        case MO_JOIN_LEFT: c = m ? m : 1; break;        // EmitUnmatchedProbe: one row with the build side NULL
-        case MO_JOIN_SEMI: c = m ? 1 : 0; break;
-        default: c = m ? 0 : 1; break;                   // anti
-        }
-        vals[i] = m ? v : 0u;
-        cnt[i] = c;
+        uint32_t v = isnull ? 0u : jt_find(tkey, tid, mask, sentinel_id, keys[i]);
+        cnt[i] = probe_row_count(&v, offsets, join_type);
+        vals[i] = v;
     }
 }
 __global__ void __launch_bounds__(kThreads) probe_emit_kernel(uint64_t n, const uint32_t *__restrict__ vals, const uint64_t *__restrict__ pos, const uint64_t *__restrict__ total,
@@ -305,6 +294,18 @@ __global__ void __launch_bounds__(kThreads) probe_emit_kernel(uint64_t n, const 
 }
 
 }  // namespace
+
+int probe_scan_emit(ThreadCtx &t, uint64_t n, const uint32_t *vals, uint64_t *cnt, const int32_t *offsets, const int32_t *sels, int join_type,
+                    uint64_t cap, int64_t *out_probe, int64_t *out_build, int64_t *count_out, int64_t *produced) {
+    uint64_t *total = (uint64_t *)arena_alloc(t, 8);
+    if (!total) return MO_RC_INTERNAL_ERROR;
+    int rc = exclusive_scan(t, cnt, n, cnt, total);
+    if (rc) return rc;
+    probe_emit_kernel<<<grid_for(n ? n : 1), kThreads, 0, t.stream>>>(n, vals, cnt, total, offsets, sels, join_type, cap, out_probe, out_build, count_out);
+    cudaEventRecord(t.kev1, t.stream);
+    MOB_LAUNCH_CHECK();
+    return read_back(t, produced, total, 8);
+}
 
 // Stable grouping of rows by their 1-based group id (0 = the row takes no part): *starts = uint64[ngroups + 1] (start of every 0-based group in
 // *rows), *rows = uint32[n] row ids, ascending inside every group, *scal[0] = how many rows have a group, scal[2] (as unsigned) != 0 = an id exceeded
@@ -423,18 +424,12 @@ int xcall_join_probe(mo_xcall_args_t *args, uint64_t len) {
     const uint64_t *kn = (const uint64_t *)st.in(args[7].pnulls, args[7].pnulls ? ((len + 63) / 64) * 8 : 0);
     uint32_t *vals = (uint32_t *)st.tmp(len * 4 + 4);
     uint64_t *cnt = (uint64_t *)st.tmp((len + 1) * 8);
-    uint64_t *total = (uint64_t *)st.tmp(8);
     if (st.failed) { st.finish(); return MO_RC_INTERNAL_ERROR; }
     cudaEventRecord(t.kev0, t.stream);
     probe_count_kernel<<<grid_for(len ? len : 1), kThreads, 0, t.stream>>>(keys, kn, len, T.key, T.id, T.mask, T.sentinel, offsets, P.join_type, vals, cnt);
     MOB_LAUNCH_CHECK();
-    rc = exclusive_scan(t, cnt, len, cnt, total);
-    if (rc) { st.finish(); return rc; }
-    probe_emit_kernel<<<grid_for(len ? len : 1), kThreads, 0, t.stream>>>(len, vals, cnt, total, offsets, sels, P.join_type, cap, out_probe, out_build, count);
-    cudaEventRecord(t.kev1, t.stream);
-    MOB_LAUNCH_CHECK();
     int64_t produced = 0;
-    rc = read_back(t, &produced, total, 8);
+    rc = probe_scan_emit(t, len, vals, cnt, offsets, sels, P.join_type, cap, out_probe, out_build, count, &produced);
     int frc = st.finish();
     if (rc) return rc;
     if ((uint64_t)produced > cap) { set_error("join probe: %lld result rows exceed the output capacity (%llu); the count is reported, call again with larger buffers", (long long)produced, (unsigned long long)cap); return MO_RC_OUT_OF_RANGE; }

@@ -28,6 +28,10 @@ int xcall_vector_unmarshal(mo_xcall_args_t *args, uint64_t len);
 int xcall_join_find(mo_xcall_args_t *args, uint64_t len);
 int xcall_join_probe(mo_xcall_args_t *args, uint64_t len);
 int xcall_group_agg(int op, int T, mo_xcall_args_t *args, uint64_t len);
+int xcall_pack_str_keys(mo_xcall_args_t *args, uint64_t len);
+int xcall_str_group_ids(mo_xcall_args_t *args, uint64_t len);
+int xcall_str_join_find(mo_xcall_args_t *args, uint64_t len);
+int xcall_str_join_probe(mo_xcall_args_t *args, uint64_t len);
 int xcall_bruteforce(mo_xcall_args_t *args, uint64_t len);
 int xcall_ivf(mo_xcall_args_t *args, uint64_t len);
 int xcall_topk_merge(mo_xcall_args_t *args, uint64_t len);
@@ -70,6 +74,10 @@ extern "C" int32_t XCall(int64_t runtimeId, int64_t funcId, uint8_t *errStr, uin
     else if (funcId == MO_XCALL_KMEANS_ELKAN_F32 || funcId == MO_XCALL_KMEANS_ELKAN_F64) rc = xcall_kmeans(funcId, a, len);
     else if (funcId == MO_XCALL_JOIN_FIND) rc = xcall_join_find(a, len);
     else if (funcId == MO_XCALL_JOIN_PROBE) rc = xcall_join_probe(a, len);
+    else if (funcId == MO_XCALL_PACK_STR_KEYS) rc = xcall_pack_str_keys(a, len);
+    else if (funcId == MO_XCALL_STR_GROUP_IDS) rc = xcall_str_group_ids(a, len);
+    else if (funcId == MO_XCALL_STR_JOIN_FIND) rc = xcall_str_join_find(a, len);
+    else if (funcId == MO_XCALL_STR_JOIN_PROBE) rc = xcall_str_join_probe(a, len);
     else if (funcId > 0x6100 && funcId <= 0x6100 + 24) rc = xcall_shuffle((int)(funcId - 0x6100), a, len);
     else if (funcId >= 0x6400 && funcId < 0x6400 + (5 << 8)) rc = xcall_group_agg((int)((funcId - 0x6400) >> 8), (int)((funcId - 0x6400) & 0xff), a, len);
     else if (funcId == MO_XCALL_Q6_MERGE) rc = xcall_q6_merge(a, len);

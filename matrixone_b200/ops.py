@@ -681,6 +681,21 @@ def normalize_l2(cells, area, length, dtype=np.float32, nulls=None):
 
 
 # ---------------------------------------------------------------------------------------------- hash join (csrc/join.cu)
+def _group_sels(groups, nbuild, ngroups):
+    """GroupSels.Insert + Finalize over the build side's group ids (JOIN_SELS): (offsets, sels), or (None, None) when every build row has its own
+    group or none has one -- Finalize keeps no sels then (joinMapMsg.go:83-89)"""
+    if ngroups == nbuild:
+        return None, None
+    offsets = np.zeros(ngroups + 2, dtype=np.int32)
+    sels = np.zeros(max(nbuild, 1), dtype=np.int32)
+    cnt = np.zeros(1, dtype=np.int64)
+    xcall(capi.XCALL_JOIN_SELS, [Vector(data=offsets, length=ngroups + 2), Vector(data=sels, length=nbuild), Vector(data=cnt, length=1),
+                                 Vector(data=groups, length=nbuild)], nbuild)
+    if int(cnt[0]) == 0:
+        return None, None
+    return offsets, sels[:int(cnt[0])]
+
+
 class JoinMap:
     """message.JoinMap for equality joins over <= 8-byte packed keys (pkg/vm/message/joinMapMsg.go:127-210): the build side's IntHashMap
     (GroupTable: first-seen group ids + key table) and its GroupSels.  HashOnUnique (every build row its own group) keeps no sels."""
@@ -692,16 +707,7 @@ class JoinMap:
         groups = tab.insert(k, skip)                                   # HashmapBuilder.BuildHashmap: itr.Insert (hashmap.go:340-360)
         self.ngroups = int(tab.ngroups[0])
         self.table_keys = np.ascontiguousarray(tab.keys[:max(self.ngroups, 1)])[:self.ngroups].copy() if self.ngroups else np.zeros(0, np.uint64)
-        self.offsets = self.sels = None
-        if self.ngroups != self.nbuild:                                 # GroupSels.Finalize keeps sels only when some group has != 1 row (joinMapMsg.go:83-89)
-            self.offsets = np.zeros(self.ngroups + 2, dtype=np.int32)
-            self.sels = np.zeros(max(self.nbuild, 1), dtype=np.int32)
-            cnt = np.zeros(1, dtype=np.int64)
-            xcall(capi.XCALL_JOIN_SELS, [Vector(data=self.offsets, length=self.ngroups + 2), Vector(data=self.sels, length=self.nbuild), Vector(data=cnt, length=1),
-                                         Vector(data=groups, length=self.nbuild)], self.nbuild)
-            self.sels = self.sels[:int(cnt[0])]
-            if int(cnt[0]) == 0:                                       # nothing inserted (every key NULL): Finalize keeps no sels (joinMapMsg.go:83-89)
-                self.offsets = self.sels = None
+        self.offsets, self.sels = _group_sels(groups, self.nbuild, self.ngroups)
         self.prepared = False
         if prepare and self.ngroups:
             lib = capi.load_library()
@@ -744,6 +750,156 @@ class JoinMap:
         if self.prepared:
             lib = capi.load_library()
             lib.MoB200_JoinMapRelease(self.table_keys.ctypes.data)
+            self.prepared = False
+
+
+# ---------------------------------------------------------------------------------------------- keys wider than 8 bytes (csrc/strhash.cu)
+def pack_str_keys(cols, kinds, nulls=None, has_null=True, const=None, length=None, capacity=None):
+    """strHashmapIterator.encodeHashKeys (strhashmap.go:92-385): the exact StrHashMap key bytes of every row.
+    cols[k]: a fixed-width numpy column (kinds[k] = element bytes, any width >= 1) or a varlena (cells uint8[24 * n], area) pair (kinds[k] = 0);
+    nulls[k]: bitmap words or None; const[k]: column k holds one element that every row repeats (a const NULL: nulls[k] with bit 0 set).
+    Returns (offsets int64[n + 1], key bytes uint8[offsets[n]], skip bitmap words -- has_null=False only -- or None)."""
+    ncols = len(cols)
+    const = const or [False] * ncols
+    raw = []
+    n = length
+    for k, c in enumerate(cols):
+        w = int(kinds[k])
+        if w:
+            data, area = np.ascontiguousarray(c).view(np.uint8).reshape(-1), None
+        else:
+            data, area = np.ascontiguousarray(c[0], dtype=np.uint8).reshape(-1), np.ascontiguousarray(c[1], dtype=np.uint8).reshape(-1)
+        if n is None and not const[k]:
+            n = data.nbytes // (w or 24)
+        raw.append((data, area))
+    n = n if n is not None else 1
+    vecs = [Vector(data=d, area=a, nulls=None if nulls is None else nulls[k], length=1 if const[k] else n) for k, (d, a) in enumerate(raw)]
+    prm = capi.StrKeyParams(ncols, 1 if has_null else 0)
+    for k, w in enumerate(kinds):
+        prm.width[k] = int(w)
+    offsets = np.zeros(n + 1, dtype=np.int64)
+    skip = None if has_null else np.zeros((n + 63) // 64, dtype=np.uint64)
+    cap = capacity if capacity is not None else 24 * n + 64
+    while True:
+        kb = np.zeros(max(cap, 1), dtype=np.uint8)
+        rc, msg = xcall(capi.XCALL_PACK_STR_KEYS, [Vector(data=offsets, nulls=skip, length=n), Vector(data=kb, length=cap), _params_vec(prm)] + vecs, n,
+                        raise_on_error=False)
+        if rc == capi.RC_OUT_OF_RANGE and capacity is None:          # offsets[n] holds the bytes needed: size the buffer and ask again
+            cap = int(offsets[n])
+            continue
+        if rc:
+            raise capi.MoError(rc, msg)
+        return offsets, kb[:int(offsets[n])], skip
+
+
+class StrGroupTable:
+    """StrHashMap as the group operator sees it: insert(packed keys) -> 1-based group ids in first-seen order.  The key table (offsets + bytes,
+    key of group g at bytes[offsets[g - 1] : offsets[g]]) persists across batches and grows when a batch does not fit."""
+
+    def __init__(self, capacity=1024, byte_capacity=None):
+        capacity = max(int(capacity), 1)
+        self.offsets = np.zeros(capacity + 1, dtype=np.int64)
+        self.bytes = np.zeros(max(int(byte_capacity if byte_capacity is not None else 32 * capacity), 16), dtype=np.uint8)
+        self.state = np.zeros(4, dtype=np.int64)      # {ngroups, key bytes used, groups needed, bytes needed}
+
+    @property
+    def ngroups(self):
+        return int(self.state[0])
+
+    def _grow(self, groups, nbytes):
+        ng, used = self.ngroups, int(self.state[1])
+        if groups > self.offsets.shape[0] - 1:
+            off = np.zeros(max(groups, 2 * (self.offsets.shape[0] - 1)) + 1, dtype=np.int64)
+            off[:ng + 1] = self.offsets[:ng + 1]
+            self.offsets = off
+        if nbytes > self.bytes.shape[0]:
+            b = np.zeros(max(nbytes, 2 * self.bytes.shape[0]), dtype=np.uint8)
+            b[:used] = self.bytes[:used]
+            self.bytes = b
+
+    def insert(self, offsets, key_bytes, skip=None):
+        off = np.ascontiguousarray(offsets, dtype=np.int64)
+        kb = np.ascontiguousarray(key_bytes, dtype=np.uint8)
+        n = off.shape[0] - 1
+        groups = np.zeros(n, dtype=np.uint64)
+        while True:
+            rc, msg = xcall(capi.XCALL_STR_GROUP_IDS, [Vector(data=groups, length=n), Vector(data=self.state, length=4),
+                                                       Vector(data=self.offsets, length=self.offsets.shape[0]), Vector(data=self.bytes, length=self.bytes.shape[0]),
+                                                       Vector(data=off, nulls=skip, length=n), Vector(data=kb, length=kb.shape[0])], n, raise_on_error=False)
+            if rc == capi.RC_OUT_OF_RANGE:                            # the table is unchanged and the sizes are reported: grow and repeat
+                self._grow(int(self.state[2]), int(self.state[3]))
+                continue
+            if rc:
+                raise capi.MoError(rc, msg)
+            return groups
+
+    def table(self):
+        """(offsets int64[ngroups + 1], bytes) of the groups so far, copies"""
+        ng = self.ngroups
+        return self.offsets[:ng + 1].copy(), self.bytes[:int(self.state[1])].copy()
+
+    def key(self, g):
+        return self.bytes[self.offsets[g - 1]:self.offsets[g]].tobytes()
+
+
+class StrJoinMap:
+    """message.JoinMap for equality joins over StrHashMap keys (the build side's packed keys): first-seen group ids + key table (StrGroupTable)
+    and the GroupSels of JOIN_SELS.  find / probe take the probe side's packed keys (pack_str_keys)."""
+
+    def __init__(self, build_offsets, build_bytes, skip=None, prepare=True):
+        off = np.ascontiguousarray(build_offsets, dtype=np.int64)
+        self.nbuild = off.shape[0] - 1
+        tab = StrGroupTable(max(self.nbuild, 1), max(int(off[-1]), 16))
+        groups = tab.insert(off, build_bytes, skip)                    # HashmapBuilder.BuildHashmap: itr.Insert (hashmap.go:340-360)
+        self.ngroups = tab.ngroups
+        self.key_offsets, self.key_bytes = tab.table()
+        self.offsets, self.sels = _group_sels(groups, self.nbuild, self.ngroups)
+        self.prepared = False
+        if prepare and self.ngroups:
+            lib = capi.load_library()
+            capi.check(lib.MoB200_StrJoinMapPrepare(self.key_offsets.ctypes.data, self.key_bytes.ctypes.data, self.ngroups), lib)
+            self.prepared = True
+
+    def hash_on_unique(self):
+        return self.offsets is None
+
+    def _table(self):
+        return [Vector(data=self.key_offsets, length=self.ngroups + 1), Vector(data=self.key_bytes, length=self.key_bytes.shape[0])]
+
+    def find(self, offsets, key_bytes, skip=None):
+        """strHashmapIterator.Find: 1-based group id per probe key, 0 = no match (or a skipped row)"""
+        off = np.ascontiguousarray(offsets, dtype=np.int64)
+        n = off.shape[0] - 1
+        vals = np.zeros(n, dtype=np.uint64)
+        xcall(capi.XCALL_STR_JOIN_FIND, [Vector(data=vals, length=n)] + self._table() +
+              [Vector(data=off, nulls=skip, length=n), Vector(data=np.ascontiguousarray(key_bytes, dtype=np.uint8))], n)
+        return vals
+
+    def probe(self, offsets, key_bytes, join_type=capi.JOIN_INNER, skip=None, capacity=None):
+        """(probe rows, build rows) of the join result in the reference's emission order, as JoinMap.probe"""
+        off = np.ascontiguousarray(offsets, dtype=np.int64)
+        kb = np.ascontiguousarray(key_bytes, dtype=np.uint8)
+        n = off.shape[0] - 1
+        cap = capacity if capacity is not None else max(2 * n, 1024)
+        prm = np.array([join_type, 0], dtype=np.int32)
+        while True:
+            op, ob, cnt = np.zeros(cap, np.int64), np.zeros(cap, np.int64), np.zeros(1, np.int64)
+            vecs = [Vector(data=op, length=cap), Vector(data=ob, length=cap), Vector(data=cnt, length=1), Vector(data=prm.view(np.uint8), length=1)] + self._table() + [
+                Vector(data=self.offsets, length=self.ngroups + 2) if self.offsets is not None else Vector(length=0),
+                Vector(data=self.sels, length=len(self.sels)) if self.sels is not None else Vector(length=0),
+                Vector(data=off, nulls=skip, length=n), Vector(data=kb, length=kb.shape[0])]
+            rc, msg = xcall(capi.XCALL_STR_JOIN_PROBE, vecs, n, raise_on_error=False)
+            if rc == capi.RC_OUT_OF_RANGE and capacity is None:
+                cap = int(cnt[0])
+                continue
+            if rc:
+                raise capi.MoError(rc, msg)
+            return op[:int(cnt[0])], ob[:int(cnt[0])]
+
+    def release(self):
+        if self.prepared:
+            lib = capi.load_library()
+            lib.MoB200_StrJoinMapRelease(self.key_offsets.ctypes.data)
             self.prepared = False
 
 
